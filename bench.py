@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the set-abstraction encoder hot path: event-windows per second.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One *step* is one forward of the encoder stack sa1 -> sa2 -> sa3 (TEHNet.py:172-181) over
 one batch of synthetic event windows ([B, 5, 2048] float32, ev2hands_b200.synth).  At N=1
@@ -19,6 +19,10 @@ Printed JSON (one line, rank 0): the driver contract plus
 
 --impl reference times the CPU oracle port of the reference (oracle/sa_oracle.py, the
 reference's algorithm op for op; /root/reference itself does not exist on the GPU box).
+
+--dump-outputs DIR writes the per-window features of the last timed step to DIR/features.npy
+(float32 [B, 1024]; one features_rank<r>.npy per rank on several GPUs).  The inputs and weights
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -41,6 +45,20 @@ N_POINTS = 2048
 MLP_MAC_PER_WINDOW = 4_468_080_640
 ALGO_BYTES_PER_WINDOW = 1_900_000       # compulsory HBM traffic per window (SURVEY.md 8d)
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_BYTES_MAX = 64_000_000             # --dump-outputs: all files of one run together
+
+
+def dump_features(directory: str, feats: np.ndarray, name: str = "features", budget: int = DUMP_BYTES_MAX):
+    """Writes feats [B, C] as <directory>/<name>.npy in float32.  A batch larger than the budget keeps a fixed, seeded
+    sample of its windows (the same for every build), and <name>_windows.npy (float64) holds their numbers."""
+    feats = np.ascontiguousarray(feats, dtype=np.float32)
+    os.makedirs(directory, exist_ok=True)
+    if feats.nbytes > budget - 4096:                       # 4 KiB for the .npy headers
+        n_keep = (budget - 4096) // (feats[0].nbytes + 8)
+        keep = np.sort(np.random.RandomState(0).choice(len(feats), n_keep, replace=False))
+        np.save(os.path.join(directory, name + "_windows.npy"), keep.astype(np.float64))
+        feats = feats[keep]
+    np.save(os.path.join(directory, name + ".npy"), feats)
 
 
 def load_peaks():
@@ -118,7 +136,8 @@ def oracle_states():
 
 def time_cpu_oracle(n_windows: int, reps: int, warmup: int, device: str = "cpu", threads: int | None = None):
     """Reference algorithm (oracle port) on the host - or, device="cuda", the same stock-PyTorch ops on the GPU,
-    the comparator SURVEY.md 8d asks for since the reference ships no kernels: returns (windows/s, threads, seconds per rep)."""
+    the comparator SURVEY.md 8d asks for since the reference ships no kernels: returns (windows/s, threads, seconds per rep,
+    features [n_windows, 1024] of the last rep)."""
     from ev2hands_b200 import synth
     from oracle import sa_oracle
     threads = threads or os.cpu_count() or 1
@@ -138,14 +157,14 @@ def time_cpu_oracle(n_windows: int, reps: int, warmup: int, device: str = "cpu",
             if cuda:
                 torch.cuda.synchronize()
             t0 = time.perf_counter()
-            sa_oracle.encoder_forward(states, synth.ENCODER_SPECS, ev, starts)
+            out = sa_oracle.encoder_forward(states, synth.ENCODER_SPECS, ev, starts)
             if cuda:
                 torch.cuda.synchronize()
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
     torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old_tf32
-    return n_windows / (sum(times) / len(times)), threads, times
+    return n_windows / (sum(times) / len(times)), threads, times, out.squeeze(-1)
 
 
 def run_reference_arm(args):
@@ -154,7 +173,9 @@ def run_reference_arm(args):
         return 0
     sample = 4
     t0 = time.perf_counter()
-    wps, threads, times = time_cpu_oracle(sample, max(1, args.steps), max(1, min(args.warmup, 2)))
+    wps, threads, times, feats = time_cpu_oracle(sample, args.steps, max(1, min(args.warmup, 2)))
+    if args.dump_outputs:
+        dump_features(args.dump_outputs, feats.float().cpu().numpy())
     line = {
         "impl": "reference", "metric": "encoder event-windows/s", "value": wps, "unit": "windows/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -428,6 +449,9 @@ def run_ours(args):
     # of the timed steps' result (fixed windows and FPS starts): taken now, because a replayed graph returns its static
     # output buffer and the end-to-end leg below overwrites it with the result of randomly drawn start indices
     headline_checksum = float(out.double().sum().item())
+    if args.dump_outputs:
+        dump_features(args.dump_outputs, out.float().cpu().numpy(), "features" if world == 1 else "features_rank%d" % rank,
+                      DUMP_BYTES_MAX // world)
 
     # rows the fused kernel evaluated in the headline step / dense B*S*K rows, per scale (read now: the later legs run
     # other batch sizes through the same modules)
@@ -842,7 +866,7 @@ def run_ours(args):
         except Exception as exc:      # noqa: BLE001
             print("bench.py: CPU window recipe failed (%s)" % exc, file=sys.stderr)
     if world == 1 and not args.no_cpu_baseline:
-        wps, threads, times = time_cpu_oracle(4, 3, 1)
+        wps, threads, times, _ = time_cpu_oracle(4, 3, 1)
         line["cpu_baseline"] = {"value": wps, "unit": "windows/s", "cores": threads, "kind": "port",
                                 "sample": "4 windows per run, 1 warm-up + 3 timed runs of oracle/sa_oracle.py (torch CPU, "
                                           "the reference's algorithm op for op)"}
@@ -851,14 +875,14 @@ def run_ours(args):
         try:
             cfg1 = {}
             for label, nthr in (("all_threads", os.cpu_count() or 1), ("one_thread", 1)):
-                _, _, t1 = time_cpu_oracle(1, 5, 2, threads=nthr)
+                _, _, t1, _ = time_cpu_oracle(1, 5, 2, threads=nthr)
                 cfg1[label] = {"threads": nthr, "windows_per_s_best": 1.0 / min(t1), "windows_per_s_median": 1.0 / float(np.median(t1)),
                                "ms_min": 1e3 * min(t1), "ms_median": 1e3 * float(np.median(t1))}
             line["cpu_baseline"]["cfg1_batch1"] = cfg1
         except Exception as exc:      # noqa: BLE001
             line["cpu_baseline"]["cfg1_batch1"] = {"unavailable": str(exc)[:200]}
         try:      # the same stock-PyTorch ops on this GPU (the reference ships no kernels): informational comparator
-            gwps, _, _ = time_cpu_oracle(WINDOWS_PER_GPU, 2, 1, device="cuda")
+            gwps, _, _, _ = time_cpu_oracle(WINDOWS_PER_GPU, 2, 1, device="cuda")
             line["torch_gpu_baseline"] = {"value": gwps, "unit": "windows/s", "kind": "port",
                                           "sample": "64 windows per run (the workload's batch), 1 warm-up + 2 timed runs of oracle/sa_oracle.py on cuda:0 "
                                                     "(stock PyTorch fp32 ops, Python FPS loop, materialised distance matrices)"}
@@ -870,12 +894,21 @@ def run_ours(args):
     return 0
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % v)
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps of the headline")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the features the last timed step computed to DIR/features.npy (float32)")
     ap.add_argument("--windows-per-gpu", type=int, default=WINDOWS_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", dest="configs", action="store_false",

@@ -277,6 +277,15 @@ def dump_state_dict_layout():
     out["fp1"] = {k: list(v.shape) for k, v in net.fp1.state_dict().items()}
     with open(os.path.join(HERE, "state_dict_layout.json"), "w") as f:
         json.dump(out, f, indent=1, sort_keys=True)
+    write_tehnet_layout(net)
+
+
+def write_tehnet_layout(net):
+    """The whole network's state_dict in order, one [name, shape, dtype] per line -> tests/golden/tehnet_layout.json."""
+    import json
+    rows = [json.dumps([k, list(v.shape), str(v.dtype).replace("torch.", "")]) for k, v in net.state_dict().items()]
+    with open(os.path.join(HERE, "tehnet_layout.json"), "w") as f:
+        f.write("[\n" + ",\n".join(rows) + "\n]\n")
 
 
 if __name__ == "__main__":

@@ -723,13 +723,15 @@ def test_point_records_kernel(b, n, d):
     assert torch.equal(got, want)
 
 
-def test_bench_prints_the_contract_line():
-    """one short `bench.py` run through the driver's command line: ONE JSON line with the keys the contract names"""
+def test_bench_prints_the_contract_line(tmp_path):
+    """one short `bench.py` run through the driver's command line: ONE JSON line with the keys the contract names;
+    --dump-outputs writes the features of the last timed step, the ones the checksum sums"""
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "3",
-                          "--no-configs", "--no-raw-events", "--no-cpu-baseline"], capture_output=True, text=True, timeout=900, cwd=root)
+                          "--no-configs", "--no-raw-events", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "dump")],
+                         capture_output=True, text=True, timeout=900, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -743,6 +745,10 @@ def test_bench_prints_the_contract_line():
     r = d["roofline"]
     assert r["bound"] == "tensor" and 0 < r["frac"] < 1 and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-6
     assert abs(d["ms_per_step"] * d["value"] / 1e3 - 64) < 0.5          # 64 windows per step
+    assert os.listdir(tmp_path / "dump") == ["features.npy"]
+    feats = np.load(tmp_path / "dump" / "features.npy")
+    assert feats.dtype == np.float32 and feats.shape == (64, 1024) and np.isfinite(feats).all()
+    assert abs(feats.astype(np.float64).sum() - d["checksum"]) <= 1e-9 * max(abs(d["checksum"]), 1.0)
 
 
 @pytest.mark.parametrize("m,cout,cin,ld_x", [(4096, 64, 8, 8), (100000, 96, 64, 64), (33333, 128, 323, 324), (5000, 196, 128, 128),

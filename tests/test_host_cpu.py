@@ -164,7 +164,10 @@ def test_header_is_plain_c_and_links_from_c(tmp_path):
     assert int(out[0]) >= 100 and int(out[1]) == len(names)
 
 
-REF_MODEL_DIR = "/root/reference/src/Ev2Hands/model"
+# The original Ev2Hands project is not part of this repository: the test that runs its own TEHNet.py reads it from the
+# checkout EV2HANDS_REFERENCE names and skips without one.
+REF_MODEL_DIR = os.path.join(os.environ.get("EV2HANDS_REFERENCE", ""), "src", "Ev2Hands", "model")
+HAVE_REF = bool(os.environ.get("EV2HANDS_REFERENCE")) and os.path.isdir(REF_MODEL_DIR)
 
 
 def _load_tehnet(pkg_name, pointnet2_module=None):
@@ -186,7 +189,7 @@ def _load_tehnet(pkg_name, pointnet2_module=None):
     return mod
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MODEL_DIR), reason="the reference tree exists in the build container only")
+@pytest.mark.skipif(not HAVE_REF, reason="needs a checkout of the original Ev2Hands project in EV2HANDS_REFERENCE")
 def test_one_line_change_builds_the_real_tehnet_and_loads_its_checkpoint(monkeypatch):
     """SURVEY 7 step 6 / INTEGRATION.md: the UNMODIFIED reference TEHNet.py with line 6 pointed at ev2hands_b200
     constructs (TEHNet.__init__ :115-166, both MANORegressors :43-44 included), has the stock net's state_dict
@@ -217,30 +220,51 @@ def test_one_line_change_builds_the_real_tehnet_and_loads_its_checkpoint(monkeyp
         patched.eval()(torch.zeros(1, 5, 2048), {"left": None, "right": None})
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MODEL_DIR), reason="the reference tree exists in the build container only")
-def test_tehnet_wiring_has_the_reference_checkpoint_layout_and_attention_matches(monkeypatch):
-    """ev2hands_b200.tehnet.TEHNet (the wiring the training configuration and rows N2 / N4 run on): same state_dict
-    names, shapes and dtypes as the reference's TEHNet, strict loads in both directions, and AttentionBlock equal to
-    the reference's (TEHNet.py:9-27) on random inputs."""
+def test_tehnet_wiring_has_the_reference_checkpoint_layout_and_attention_matches(monkeypatch, golden):
+    """ev2hands_b200.tehnet.TEHNet (the wiring the training configuration and rows N2 / N4 run on): the state_dict
+    names in order, shapes and dtypes of the reference's TEHNet (tests/golden/tehnet_layout.json), a strict load of a
+    checkpoint of that layout, and the classifier, query convolutions and AttentionBlock (TEHNet.py:9-27) equal to the
+    reference's outputs on the CPU (tests/golden/heads.npz)."""
     monkeypatch.setenv("ERPC", "1")
     from ev2hands_b200 import tehnet
-    ref_mod = _load_tehnet("refmodel_stock2")
-    ref = ref_mod.TEHNet(n_pose_params=6)
+    with open(os.path.join(ROOT, "tests", "golden", "tehnet_layout.json")) as f:
+        layout = [(k, tuple(s), d) for k, s, d in json.load(f)]
     ours = tehnet.TEHNet(n_pose_params=6)
-    a, b = ref.state_dict(), ours.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    assert all(a[k].shape == b[k].shape and a[k].dtype == b[k].dtype for k in a)
-    ours.load_state_dict(a, strict=True)
-    ref.load_state_dict(ours.state_dict(), strict=True)
-    torch.manual_seed(1)
-    key, val, qry = torch.randn(2, 4, 64), torch.randn(2, 256, 64), torch.randn(2, 256, 64)
-    assert torch.allclose(tehnet.AttentionBlock()(key, val, qry), ref_mod.AttentionBlock()(key, val, qry), rtol=1e-5, atol=1e-6)
-    # the heads after the encoder (classifier, query convs, attention) agree with the reference's on CPU
-    ref.eval(), ours.eval()
-    feats = torch.randn(2, 256, 64)
+    assert [(k, tuple(v.shape), str(v.dtype).replace("torch.", "")) for k, v in ours.state_dict().items()] == layout
+    # the stored layout agrees with what the reference wrote or loaded itself: its modules' layouts
+    # (state_dict_layout.json) and the decoder and head weights of the golden vectors
+    shapes = {k: list(s) for k, s, _ in layout}
+    parts = json.load(open(os.path.join(ROOT, "tests", "golden", "state_dict_layout.json")))
+    g = golden("heads")
+    head_state = synth.random_head_state(seed=int(g["weight_seed"]))
+    for name, prefixes in (("encoder.sa1", ["sa1"]), ("encoder.sa2", ["sa2"]), ("encoder.sa3", ["sa3"]), ("fp1", ["fp1"]),
+                           ("regressor.sa1", ["left_mano_regressor.sa1", "right_mano_regressor.sa1"]),
+                           ("regressor.sa2", ["left_mano_regressor.sa2", "right_mano_regressor.sa2"])):
+        for p in prefixes:
+            assert {k[len(p) + 1:]: s for k, s in shapes.items() if k.startswith(p + ".")} == parts[name], p
+    for n in ("fp3", "fp2"):
+        want = {k: list(np.shape(v)) for k, v in synth.random_state_for(synth.DECODER_SPECS[n], seed=0).items()}
+        assert {k[len(n) + 1:]: s for k, s in shapes.items() if k.startswith(n + ".")} == want, n
+    assert all(shapes[k] == list(np.shape(v)) for k, v in head_state.items())
+    gen = torch.Generator().manual_seed(1)
+    ckpt = {k: (torch.randn(s, generator=gen) if d.startswith("float") else torch.randint(0, 100, s, generator=gen)).to(getattr(torch, d))
+            for k, s, d in layout}
+    ours.load_state_dict(ckpt, strict=True)
+    assert all(torch.equal(v, ckpt[k]) for k, v in ours.state_dict().items())
+    # the heads after the decoder, with the reference's golden weights and features
+    res = ours.load_state_dict({k: torch.from_numpy(np.asarray(v)) for k, v in head_state.items()}, strict=False)
+    assert not res.unexpected_keys
+    ours.eval()
+    feat = torch.from_numpy(np.random.RandomState(int(g["feature_seed"])).randn(2, 256, 2048).astype(np.float32))
     with torch.no_grad():
-        for name in ("classifier", "left_query_conv", "right_query_conv"):
-            assert torch.equal(getattr(ours, name)(feats), getattr(ref, name)(feats)), name
+        seg = ours.classifier(feat)
+        lq, rq = ours.left_query_conv(feat), ours.right_query_conv(feat)
+        got = {"seg_out": seg, "left_query_every8": lq[:, :, ::8],
+               "left_features": ours.attention_block(seg, feat, lq), "right_features": ours.attention_block(seg, feat, rq)}
+    for name, t in got.items():
+        want = torch.from_numpy(g[name])
+        # same modules, same weights: equal up to the last bits another CPU's summation order may change
+        assert torch.allclose(t, want, rtol=1e-5, atol=1e-6 * float(want.abs().max())), name
 
 
 def test_standin_mano_layer_and_training_losses():
@@ -275,15 +299,19 @@ def test_standin_mano_layer_and_training_losses():
     assert outs["class_logits"].grad.abs().sum() > 0
 
 
-def test_bench_reference_arm_prints_the_contract_line():
+def test_bench_reference_arm_prints_the_contract_line(tmp_path):
     """`bench.py --impl reference` (the arm the driver times beside ours) runs the oracle port on the host and prints ONE
-    JSON line with the keys the driver reads; no GPU, no kernel of this repo."""
+    JSON line with the keys the driver reads; no GPU, no kernel of this repo.  --dump-outputs writes the last step's
+    features; --steps below 1 is refused."""
     import json
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1"],
+    bad = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "0"],
                          capture_output=True, text=True, timeout=600, cwd=root)
+    assert bad.returncode != 0 and "--steps" in bad.stderr
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                          "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -293,3 +321,28 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": "windows/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d.get("gpu_launches", 0) == 0
+    assert os.listdir(tmp_path / "dump") == ["features.npy"]
+    feats = np.load(tmp_path / "dump" / "features.npy")
+    assert feats.dtype == np.float32 and feats.shape == (4, 1024) and np.isfinite(feats).all()
+
+
+def test_bench_dump_keeps_a_fixed_sample_of_a_large_batch(tmp_path):
+    """bench.py's --dump-outputs writer: a batch over the size budget is cut to the same seeded sample of windows every
+    time, with the window numbers beside it, and the files stay within the budget."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    feats = np.random.RandomState(3).randn(500, 1024).astype(np.float32)
+    for d in ("a", "b"):
+        bench.dump_features(str(tmp_path / d), feats, budget=400_000)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 400_000
+    rows = np.load(tmp_path / "a" / "features_windows.npy")
+    got = np.load(tmp_path / "a" / "features.npy")
+    assert rows.dtype == np.float64 and len(rows) == len(got) > 0 and (np.diff(rows) > 0).all()
+    assert np.array_equal(got, feats[rows.astype(np.int64)])
+    for f in ("features.npy", "features_windows.npy"):
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes()
+    bench.dump_features(str(tmp_path / "small"), feats[:8])
+    assert os.listdir(tmp_path / "small") == ["features.npy"]
+    assert np.array_equal(np.load(tmp_path / "small" / "features.npy"), feats[:8])
