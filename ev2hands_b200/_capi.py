@@ -38,9 +38,9 @@ _SIGNATURES = {
     "ev2h_tc_pack_weights": [c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp],
     "ev2h_tc_pack_weights_kc": [c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp],
     "ev2h_sa_msg_fused_kc": [c_int, ctypes.POINTER(ctypes.c_int32)],
-    "ev2h_linear_relu_tc": [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp],
+    "ev2h_linear_relu_tc": [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp],
     "ev2h_tc_set_debug": [c_int],
-    "ev2h_linear_tc": [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_vp],
+    "ev2h_linear_tc": [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp],
     "ev2h_fused_set_debug_buffer": [c_vp],
     "ev2h_linear_f32": [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_vp],
     "ev2h_sa_msg_fused_tc": [c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_int,
@@ -71,7 +71,8 @@ _SIGNATURES = {
     "ev2h_ball_query_compact_range_f32": [c_vp, c_i64, c_i64, c_i64, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                           ctypes.POINTER(c_f), ctypes.POINTER(ctypes.c_int32), c_vp, c_vp, c_vp,
                                           ctypes.POINTER(c_vp), ctypes.POINTER(c_vp), c_vp, c_vp],
-    "ev2h_conv1d_tc": [c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp],
+    "ev2h_conv1d_tc": [c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp,
+                       c_vp],
     "ev2h_class_attention_f32": [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, c_vp, c_vp],
     "ev2h_group_max_f32": [c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp],
     "ev2h_group_max_bwd_f32": [c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp],
@@ -473,7 +474,9 @@ def tc_supported(Cout: int, pool_rows: int) -> bool:
 
 def tc_pack(wt: torch.Tensor, Cin: int, Cout: int, mode: int, kc: int = 32, row_align: int = 16) -> torch.Tensor:
     """folded wt [Cin_pad, Cout_pad] -> packed shared-memory images (uint8 buffer) for `mode`,
-    `kc` input channels per image, image rows padded to a multiple of `row_align`."""
+    `kc` input channels per image, image rows padded to a multiple of `row_align`.
+    TC_F16X3: a weight outside the fp16 range (or NaN) raises the device's range flag - a BatchNorm with a tiny
+    running variance and a large gamma folds into such weights (checked on the device, no synchronisation)."""
     n = lib().ev2h_tc_packed_bytes_kc(Cin, Cout, mode, kc, row_align)
     if n <= 0:
         raise RuntimeError("ev2h_tc_packed_bytes_kc(%d, %d, %d, %d, %d) failed" % (Cin, Cout, mode, kc, row_align))
@@ -482,6 +485,8 @@ def tc_pack(wt: torch.Tensor, Cin: int, Cout: int, mode: int, kc: int = 32, row_
         with _timed("ev2h_tc_pack_weights"):
             _check(lib().ev2h_tc_pack_weights_kc(_p(wt), wt.shape[1], Cin, Cout, mode, kc, row_align, _p(packed), _stream(wt)),
                    "ev2h_tc_pack_weights_kc")
+        if mode == TC_F16X3:
+            range_flag(wt.device).bitwise_or_((~(wt.abs().amax() < 65520.0)).to(torch.int32))
     return packed
 
 
@@ -491,18 +496,25 @@ def fused_kc(mode: int, couts) -> int:
     return lib().ev2h_sa_msg_fused_kc(mode, arr)
 
 
+def _f16_flag(t, mode):
+    """the device's range flag for the fp16-split mode (the kernels track their inputs' range there), else NULL"""
+    return range_flag(t.device) if mode == TC_F16X3 else None
+
+
 def linear_relu_tc(x, M, ld_x, Cin, packed, bias, Cout, pool_rows, y, ld_y, y_col_off, mode):
+    flag = _f16_flag(x, mode)
     with torch.cuda.device(x.device):
         with _timed("ev2h_linear_relu_tc"):
             _check(lib().ev2h_linear_relu_tc(_p(x), M, ld_x, Cin, _p(packed), _p(bias), Cout, pool_rows, _p(y), ld_y,
-                                             y_col_off, mode, _stream(x)), "ev2h_linear_relu_tc")
+                                             y_col_off, mode, _p(flag), _stream(x)), "ev2h_linear_relu_tc")
 
 
 def linear_tc_no_relu(x, M, ld_x, Cin, packed, bias, Cout, y, ld_y, y_col_off, mode):
+    flag = _f16_flag(x, mode)
     with torch.cuda.device(x.device):
         with _timed("ev2h_linear_tc"):
             _check(lib().ev2h_linear_tc(_p(x), M, ld_x, Cin, _p(packed), _p(bias), Cout, _p(y), ld_y, y_col_off, mode,
-                                        _stream(x)), "ev2h_linear_tc")
+                                        _p(flag), _stream(x)), "ev2h_linear_tc")
 
 
 def linear_no_relu(x, M, ld_x, Cin, wt, bias, Cout, y, ld_y, y_col_off=0):
@@ -514,10 +526,12 @@ def linear_no_relu(x, M, ld_x, Cin, wt, bias, Cout, y, ld_y, y_col_off=0):
 
 def conv1d_tc(x_rows, M, ld_x, Cin, taps, rows_per_seq, packed, bias, Cout, relu, post_scale, post_shift, y, ld_y, y_col_off, mode):
     """Conv1d (kernel size taps, zero padding taps // 2) over point-major rows [+ ReLU] [+ per-channel affine]."""
+    flag = _f16_flag(x_rows, mode)
     with torch.cuda.device(x_rows.device):
         with _timed("ev2h_conv1d_tc"):
             _check(lib().ev2h_conv1d_tc(_p(x_rows), M, ld_x, Cin, taps, rows_per_seq, _p(packed), _p(bias), Cout, 1 if relu else 0,
-                                        _p(post_scale), _p(post_shift), _p(y), ld_y, y_col_off, mode, _stream(x_rows)), "ev2h_conv1d_tc")
+                                        _p(post_scale), _p(post_shift), _p(y), ld_y, y_col_off, mode, _p(flag), _stream(x_rows)),
+                   "ev2h_conv1d_tc")
 
 
 def class_attention(key_rows, ld_k, query_rows, ld_q, value_rows, ld_v, B, N, C, D, scale):
@@ -548,7 +562,9 @@ _range_flags = {}
 
 
 def range_flag(device) -> torch.Tensor:
-    """int32 [1] on `device`: bit 0 is set by the fused kernel when an fp16-split operand overflowed (TC_F16X3)."""
+    """int32 [1] on `device`: bit 0 is set when an operand of the fp16 split (TC_F16X3) left the fp16 range or was NaN -
+    by the fused kernel and the per-layer kernels (ev2h_linear_tc, ev2h_linear_relu_tc, ev2h_conv1d_tc) for their
+    activation inputs, and by tc_pack for the weights it packs."""
     device = torch.device(device)
     if device.index is None:
         device = torch.device("cuda", torch.cuda.current_device())
@@ -559,7 +575,7 @@ def range_flag(device) -> torch.Tensor:
 
 
 def check_numeric_range(device="cuda", reset: bool = True) -> bool:
-    """True if no fused launch on `device` saw an activation outside the fp16 range since the last reset
+    """True if no fp16-split (TC_F16X3) kernel or weight pack on `device` saw an operand outside the fp16 range since the last reset
     (synchronises; call it at a checkpoint, not per step).  Raise-free so callers decide what to do."""
     t = range_flag(device)
     ok = int(t.item()) == 0

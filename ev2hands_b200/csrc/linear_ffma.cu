@@ -21,6 +21,17 @@ __device__ __forceinline__ void atomic_max_nonneg(float *addr, float v) {
     atomicMax(reinterpret_cast<int *>(addr), __float_as_int(v));
 }
 
+// x[k .. k+3] with the channels from Cin on zeroed: columns Cin .. ld_x - 1 are padding and must not enter the product
+// (a NaN or Inf there would survive the zero weight rows), whatever they hold
+__device__ __forceinline__ float4 tail_masked(float4 v, int k, int Cin) {
+    if (k + 4 > Cin) {
+        if (k + 1 >= Cin) v.y = 0.f;
+        if (k + 2 >= Cin) v.z = 0.f;
+        if (k + 3 >= Cin) v.w = 0.f;
+    }
+    return v;
+}
+
 __global__ void __launch_bounds__(LIN_THREADS, 2)
 linear_relu_kernel(const float *__restrict__ x, int64_t M, int ld_x, int Cin,
                    const float *__restrict__ wt, int ld_w, const float *__restrict__ bias,
@@ -46,8 +57,8 @@ linear_relu_kernel(const float *__restrict__ x, int64_t M, int ld_x, int Cin,
     auto load_tiles = [&](int k0) {
         xa = xb = make_float4(0.f, 0.f, 0.f, 0.f);
         const int ka = k0 + 4 * xq, kb = k0 + 4 * (xq + 2);
-        if (x_row_ok && ka < Cin) xa = *reinterpret_cast<const float4 *>(x_row + ka);
-        if (x_row_ok && kb < Cin) xb = *reinterpret_cast<const float4 *>(x_row + kb);
+        if (x_row_ok && ka < Cin) xa = tail_masked(*reinterpret_cast<const float4 *>(x_row + ka), ka, Cin);
+        if (x_row_ok && kb < Cin) xb = tail_masked(*reinterpret_cast<const float4 *>(x_row + kb), kb, Cin);
         wa = *reinterpret_cast<const float4 *>(wt + (int64_t)(k0 + wk) * ld_w + n0 + wc);
         wb = *reinterpret_cast<const float4 *>(wt + (int64_t)(k0 + wk + 8) * ld_w + n0 + wc);
     };

@@ -63,6 +63,7 @@ struct TcParams {
     int taps, tap_cin, rows_per_win;
     // optional per-channel affine AFTER the activation (a BatchNorm that follows the ReLU): y = act(.) * scale + shift
     const float *post_scale, *post_shift;
+    int32_t *range_flag;    // optional (F16X3): bit 0 set when an activation operand left the fp16 range or was NaN
 };
 
 // ---- weight packing: folded [Cin_pad16, ld_w] fp32 (input-channel major) -> per (n-block, stage)
@@ -174,6 +175,17 @@ linear_tc_kernel(const TcParams p) {
         // warp-wide load covers 8 rows x 64 contiguous bytes (full 32-byte sectors).
         const int lw = warp - 5, grp = lw >> 2, wq = lw & 3;
         const int l8 = lane & 7, oct = lane >> 3;
+        // Channels [tap_cin, ld_x) of a row are padding: never part of the product, whatever they hold.  A float4 that
+        // starts below tap_cin lies inside the row (ld_x is a multiple of 4); its components from tap_cin on are zeroed
+        // when the chunk is converted (not at the load: the loads of the next chunk must stay in flight).  With taps > 1,
+        // tap_cin is a multiple of 32 and a chunk never crosses it.
+        const int k_lim = p.tap_cin;
+        auto mask_tail = [&](float4 &t, int k) {
+            if (k + 1 >= k_lim) t.y = 0.f;
+            if (k + 2 >= k_lim) t.z = 0.f;
+            if (k + 3 >= k_lim) t.w = 0.f;
+        };
+        uint32_t hmax = 0;      // F16X3: running maximum of |fp16 hi word| pairs this thread wrote (range check)
         // The group's NEXT chunk is loaded into registers before the current one is converted and stored, so
         // the global-load latency of a stage overlaps the previous stage's wait / store / arrive.
         const uint32_t my_tiles = (uint32_t)((n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x);
@@ -201,7 +213,7 @@ linear_tc_kernel(const TcParams p) {
                     const int k = k_base + 4 * (oct + 4 * (i & 1));
                     bool ok;
                     const int64_t sr = src_row(m0 + row, ok);
-                    v[i] = (ok && k < p.ld_x)
+                    v[i] = (ok && k < k_lim)
                                ? __ldg(reinterpret_cast<const float4 *>(p.x + sr * (int64_t)p.ld_x + k))
                                : make_float4(0.f, 0.f, 0.f, 0.f);
                 }
@@ -213,8 +225,8 @@ linear_tc_kernel(const TcParams p) {
                     bool ok;
                     const int64_t sr = src_row(m0 + row, ok);
                     const float *src = p.x + sr * (int64_t)p.ld_x + k;
-                    v[2 * i] = (ok && k < p.ld_x) ? __ldg(reinterpret_cast<const float4 *>(src)) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    v[2 * i + 1] = (ok && k + 4 < p.ld_x) ? __ldg(reinterpret_cast<const float4 *>(src + 4)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                    v[2 * i] = (ok && k < k_lim) ? __ldg(reinterpret_cast<const float4 *>(src)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                    v[2 * i + 1] = (ok && k + 4 < k_lim) ? __ldg(reinterpret_cast<const float4 *>(src + 4)) : make_float4(0.f, 0.f, 0.f, 0.f);
                 }
             }
         };
@@ -238,6 +250,15 @@ linear_tc_kernel(const TcParams p) {
                     float4 vn[8];
                     const bool has_next = n + TC_LOADER_GROUPS < total;
                     if (has_next) issue_loads(n + TC_LOADER_GROUPS, vn);
+                    if (p.taps == 1 && (kc + 1) * TC_KC > k_lim) {      // the chunk that ends mid-way: warp-uniform branch
+                        if (MODE == TC_MODE_TF32X3) {
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) mask_tail(v[i], kc * TC_KC + 4 * (oct + 4 * (i & 1)));
+                        } else {
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) mask_tail(v[i], kc * TC_KC + 8 * oct + 4 * (i & 1));
+                        }
+                    }
                     tc::mbar_wait(empty_bar + stage, phase ^ 1);
                     uint8_t *st = ring + (size_t)stage * stage_bytes;
                     if (wq == 0 && lane == 0) {
@@ -265,6 +286,9 @@ linear_tc_kernel(const TcParams p) {
                             uint4 hb, lb;
                             tc::split_f16x2(v[2 * i].x, v[2 * i].y, hb.x, lb.x); tc::split_f16x2(v[2 * i].z, v[2 * i].w, hb.y, lb.y);
                             tc::split_f16x2(v[2 * i + 1].x, v[2 * i + 1].y, hb.z, lb.z); tc::split_f16x2(v[2 * i + 1].z, v[2 * i + 1].w, hb.w, lb.w);
+                            // inputs may be negative here (unlike the fused kernel's post-ReLU operands): sign bits off
+                            hmax = tc::max_u16x2(tc::max_u16x2(hmax, tc::max_u16x2(hb.x & 0x7fff7fffu, hb.y & 0x7fff7fffu)),
+                                                 tc::max_u16x2(hb.z & 0x7fff7fffu, hb.w & 0x7fff7fffu));
                             *reinterpret_cast<uint4 *>(st + oct * (TC_BLOCK_M * 16) + row * 16) = hb;
                             *reinterpret_cast<uint4 *>(st + A_PART + oct * (TC_BLOCK_M * 16) + row * 16) = lb;
                         }
@@ -312,6 +336,7 @@ linear_tc_kernel(const TcParams p) {
                 }
             }
         }
+        if (MODE == TC_MODE_F16X3 && p.range_flag != nullptr && tc::f16x2_overflowed(hmax)) atomicOr(p.range_flag, 1);
     } else if (warp == 4) {
         // ================================ UMMA issuer ================================
         // the whole warp walks the stages, one ELECTED lane issues: descriptors stay in uniform registers (under
@@ -538,34 +563,35 @@ extern "C" int ev2h_tc_pack_weights_kc(const float *wt, int ld_w, int Cin, int C
 }
 
 static int linear_tc_impl(const float *x, int64_t M, int ld_x, int Cin, const void *w_packed, const float *bias, int Cout,
-                          int pool_rows, float *y, int ld_y, int y_col_off, int mode, int relu, ev2h_stream_t stream,
-                          int taps = 1, int rows_per_win = 0, const float *post_scale = nullptr, const float *post_shift = nullptr);
+                          int pool_rows, float *y, int ld_y, int y_col_off, int mode, int relu, int32_t *range_flag,
+                          ev2h_stream_t stream, int taps = 1, int rows_per_win = 0, const float *post_scale = nullptr,
+                          const float *post_shift = nullptr);
 
 extern "C" int ev2h_linear_relu_tc(const float *x, int64_t M, int ld_x, int Cin, const void *w_packed,
                                    const float *bias, int Cout, int pool_rows, float *y, int ld_y, int y_col_off,
-                                   int mode, ev2h_stream_t stream) {
-    return linear_tc_impl(x, M, ld_x, Cin, w_packed, bias, Cout, pool_rows, y, ld_y, y_col_off, mode, 1, stream);
+                                   int mode, int32_t *range_flag, ev2h_stream_t stream) {
+    return linear_tc_impl(x, M, ld_x, Cin, w_packed, bias, Cout, pool_rows, y, ld_y, y_col_off, mode, 1, range_flag, stream);
 }
 
 extern "C" int ev2h_linear_tc(const float *x, int64_t M, int ld_x, int Cin, const void *w_packed, const float *bias,
-                              int Cout, float *y, int ld_y, int y_col_off, int mode, ev2h_stream_t stream) {
-    return linear_tc_impl(x, M, ld_x, Cin, w_packed, bias, Cout, 0, y, ld_y, y_col_off, mode, 0, stream);
+                              int Cout, float *y, int ld_y, int y_col_off, int mode, int32_t *range_flag, ev2h_stream_t stream) {
+    return linear_tc_impl(x, M, ld_x, Cin, w_packed, bias, Cout, 0, y, ld_y, y_col_off, mode, 0, range_flag, stream);
 }
 
 extern "C" int ev2h_conv1d_tc(const float *x_rows, int64_t M, int ld_x, int Cin, int taps, int rows_per_seq, const void *w_packed,
                               const float *bias, int Cout, int relu, const float *post_scale, const float *post_shift,
-                              float *y, int ld_y, int y_col_off, int mode, ev2h_stream_t stream) {
+                              float *y, int ld_y, int y_col_off, int mode, int32_t *range_flag, ev2h_stream_t stream) {
     using namespace ev2h;
     EV2H_REQUIRE(taps == 1 || taps == 3 || taps == 5, "ev2h_conv1d_tc: kernel size %d (supported: 1, 3, 5)", taps);
     EV2H_REQUIRE(Cin > 0 && (taps == 1 || Cin % TC_KC == 0), "ev2h_conv1d_tc: Cin=%d must be a multiple of %d for kernel sizes > 1", Cin, TC_KC);
     EV2H_REQUIRE(rows_per_seq > 0 && M % rows_per_seq == 0, "ev2h_conv1d_tc: M must be a whole number of sequences");
-    return linear_tc_impl(x_rows, M, ld_x, Cin * taps, w_packed, bias, Cout, 0, y, ld_y, y_col_off, mode, relu, stream, taps, rows_per_seq,
-                          post_scale, post_shift);
+    return linear_tc_impl(x_rows, M, ld_x, Cin * taps, w_packed, bias, Cout, 0, y, ld_y, y_col_off, mode, relu, range_flag, stream,
+                          taps, rows_per_seq, post_scale, post_shift);
 }
 
 static int linear_tc_impl(const float *x, int64_t M, int ld_x, int Cin, const void *w_packed, const float *bias, int Cout,
-                          int pool_rows, float *y, int ld_y, int y_col_off, int mode, int relu, ev2h_stream_t stream,
-                          int taps, int rows_per_win, const float *post_scale, const float *post_shift) {
+                          int pool_rows, float *y, int ld_y, int y_col_off, int mode, int relu, int32_t *range_flag,
+                          ev2h_stream_t stream, int taps, int rows_per_win, const float *post_scale, const float *post_shift) {
     using namespace ev2h;
     EV2H_REQUIRE(x && w_packed && bias && y, "ev2h_linear_relu_tc: null argument");
     EV2H_REQUIRE(M > 0 && Cin > 0 && Cout > 0, "ev2h_linear_relu_tc: bad sizes");
@@ -601,6 +627,7 @@ static int linear_tc_impl(const float *x, int64_t M, int ld_x, int Cin, const vo
     p.relu = relu;
     p.taps = taps; p.tap_cin = Cin / taps; p.rows_per_win = rows_per_win > 0 ? rows_per_win : 1;
     p.post_scale = post_scale; p.post_shift = post_shift;
+    p.range_flag = mode == TC_MODE_F16X3 ? range_flag : nullptr;
     const size_t smem = (size_t)stages * stage_bytes + tail_bytes;
 
     int dev = 0, sms = 0;

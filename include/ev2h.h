@@ -210,7 +210,8 @@ EV2H_API int ev2h_fold_conv_bn_f32(const float *conv_w, const float *conv_b, con
 /* ---- shared MLP layer on CUDA cores, fp32 ------------------------------------------
  * One 1x1-conv + folded BN + ReLU layer over M rows (pointnet2_utils.py:253-256):
  *   y[m, 0..Cout) = relu( x[m, 0..Cin) . W' + b' )
- * x is [M, ld_x] (ld_x % 4 == 0, 16-byte aligned), wt/bias come from
+ * x is [M, ld_x] (ld_x % 4 == 0, 16-byte aligned; columns Cin .. ld_x - 1 are padding
+ * and never enter the product, whatever they hold), wt/bias come from
  * ev2h_fold_conv_bn_f32.  pool_rows == 0: y is [M, ld_y].  pool_rows = K > 0 fuses
  * the max over each run of K consecutive rows (torch.max(x, 2)[0],
  * pointnet2_utils.py:257): y is [M/K, ld_y] written at column y_col_off and MUST be
@@ -240,18 +241,24 @@ EV2H_API int ev2h_linear_f32(const float *x, int64_t M, int ld_x, int Cin, const
  * written by ev2h_fold_conv_bn_f32) into the kernel's shared-memory image:
  * ev2h_tc_packed_bytes gives the buffer size, ev2h_tc_pack_weights fills it.
  * pool_rows must be 0, 32, 64 or a multiple of 128; Cout <= 256 or a multiple of 256;
- * other shapes return EV2H_ERR_UNSUPPORTED (callers use ev2h_linear_relu_f32 for those). */
+ * other shapes return EV2H_ERR_UNSUPPORTED (callers use ev2h_linear_relu_f32 for those).
+ * Columns Cin .. ld_x - 1 of x are padding and never enter the product, whatever they hold (NaN included).
+ * range_flag (device int32, may be NULL; used with EV2H_TC_F16X3 only): bit 0 is set (atomic OR, never
+ * cleared) when an input operand left the fp16 range (|x| >= 65520) or was NaN.  The caller also checks the
+ * weights it packs: the kernels see them only as fp16 pairs. */
 #define EV2H_TC_BF16 0
 #define EV2H_TC_TF32X3 1
 #define EV2H_TC_TF32_BF16C 2
 #define EV2H_TC_F16X3 3      /* x = hi + lo, w = hi + lo as fp16 pairs, three kind::f16 products: fp32-level accuracy for
-                              * |activations| < 65520 (an overflow raises the fused kernel's range flag) */
+                              * |operands| < 65520; an activation outside that range (or NaN) raises the range_flag
+                              * of every entry that takes one (per-layer and fused kernels) */
 EV2H_API int64_t ev2h_tc_packed_bytes(int Cin, int Cout, int mode);
 EV2H_API int ev2h_tc_pack_weights(const float *wt, int ld_w, int Cin, int Cout, int mode, void *packed,
                                   ev2h_stream_t stream);
 /* The tensor-core layer without the ReLU (y = x W' + b'), cf. ev2h_linear_f32. */
 EV2H_API int ev2h_linear_tc(const float *x, int64_t M, int ld_x, int Cin, const void *w_packed, const float *bias,
-                            int Cout, float *y, int ld_y, int y_col_off, int mode, ev2h_stream_t stream);
+                            int Cout, float *y, int ld_y, int y_col_off, int mode, int32_t *range_flag,
+                            ev2h_stream_t stream);
 
 /* Same with an explicit K-chunk length (16 or 32 input channels per shared-memory image;
  * ev2h_sa_msg_fused_kc tells which one the fused kernel wants) and row padding of the image:
@@ -262,7 +269,7 @@ EV2H_API int ev2h_tc_pack_weights_kc(const float *wt, int ld_w, int Cin, int Cou
                                      void *packed, ev2h_stream_t stream);
 EV2H_API int ev2h_linear_relu_tc(const float *x, int64_t M, int ld_x, int Cin, const void *w_packed,
                                  const float *bias, int Cout, int pool_rows, float *y, int ld_y,
-                                 int y_col_off, int mode, ev2h_stream_t stream);
+                                 int y_col_off, int mode, int32_t *range_flag, ev2h_stream_t stream);
 /* ---- weight gradient of a 1x1 convolution over point rows (training path) ---------------------------------
  * dW [Cout, Cin] (row-major, contiguous) = dY^T X with dY [M, ld_dy >= Cout] and X [M, ld_x >= Cin] fp32 rows - the
  * autograd of Conv2d(1x1) (pointnet2_utils.py:253-256) when the grouped tensor is kept as rows: a GEMM whose contraction
@@ -300,10 +307,11 @@ EV2H_API int ev2h_ball_query_compact_range_f32(const float *xyz, int64_t stride_
  * positions x Cin channels; y[r] = act(sum_t W_t x[r + t - taps/2] + b) * post_scale + post_shift, rows outside a
  * sequence counting as zero (the convolution's zero padding).  The shifted rows are gathered by the kernel's loaders;
  * no im2col buffer exists.  w_packed = ev2h_tc_pack_weights_kc image of the [taps * Cin, Cout] matrix whose row
- * t * Cin + ci is W[:, ci, t] (kc 32, row_align 16); post_scale / post_shift may be NULL.  taps in {1, 3, 5}. */
+ * t * Cin + ci is W[:, ci, t] (kc 32, row_align 16); post_scale / post_shift may be NULL.  taps in {1, 3, 5}.
+ * Columns Cin .. ld_x - 1 of x_rows are padding and never enter the product; range_flag as for ev2h_linear_tc. */
 EV2H_API int ev2h_conv1d_tc(const float *x_rows, int64_t M, int ld_x, int Cin, int taps, int rows_per_seq, const void *w_packed,
                             const float *bias, int Cout, int relu, const float *post_scale, const float *post_shift,
-                            float *y, int ld_y, int y_col_off, int mode, ev2h_stream_t stream);
+                            float *y, int ld_y, int y_col_off, int mode, int32_t *range_flag, ev2h_stream_t stream);
 
 /* ---- class-wise attention pooling (SURVEY.md 8f row N2) ------------------------------------------
  * Replaces AttentionBlock.forward (reference TEHNet.py:9-27): sim[b,c,d] = scale * sum_n key[b,n,c] query[b,n,d],
@@ -337,7 +345,8 @@ EV2H_API int ev2h_class_attention_f32(const float *key_rows, int ld_k, const flo
  * ev2h_tc_pack_weights_kc images (kc from ev2h_sa_msg_fused_kc), bias_host[2] their folded biases
  * (device pointers in host arrays).  out_rows [B*S, ld_out]: the pooled features of this scale
  * are written at column out_col.  mode: EV2H_TC_BF16 / EV2H_TC_TF32X3 / EV2H_TC_TF32_BF16C / EV2H_TC_F16X3.
- * range_flag (device int32, may be NULL): bit 0 is set when an EV2H_TC_F16X3 operand left the fp16 range.
+ * range_flag (device int32, may be NULL): bit 0 is set when an EV2H_TC_F16X3 activation operand left the fp16
+ * range or was NaN (the layer-1 outputs and the layer-2 activations the kernel splits itself).
  * Deviation from the reference (all modes): ReLU and the max-pool are evaluated with fmaxf / an integer atomic
  * max on zero-initialised output, so a NaN activation becomes 0 where F.relu / torch.max would propagate it. */
 EV2H_API int ev2h_sa_msg_fused_tc(

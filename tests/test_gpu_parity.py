@@ -181,7 +181,9 @@ def precision(request):
 @pytest.mark.parametrize("M,cin,widths,pool", [
     (1000, 8, [32, 32, 64], 0), (64 * 32, 8, [32, 32, 64], 32), (40 * 64, 323, [128, 196, 256], 64),
     (6 * 128, 515, [256, 512, 1024], 128), (5 * 256, 19, [40], 256), (24 * 12, 7, [130], 12), (9 * 20, 5, [33, 17], 20),
-    (300 * 128 + 128, 64, [96, 128], 128), (777, 100, [300, 48], 0)])
+    (300 * 128 + 128, 64, [96, 128], 128), (777, 100, [300, 48], 0),
+    (1000, 40, [96, 768], 0), (3 * 384, 16, [64, 128], 384), (2000, 33, [64, 32], 0), (1536, 257, [128], 64),
+    (32 * 37, 20, [48, 80], 32)])
 def test_linear_relu_stack_vs_fp64(M, cin, widths, pool, precision):
     rs = np.random.RandomState(M + cin)
     spec = dict(kind="all", in_channel=cin, mlp=widths)
