@@ -12,5 +12,5 @@ void set_error(const char *fmt, ...) {
 }
 }  // namespace ev2h
 
-extern "C" int ev2h_version(void) { return 101; }
+extern "C" int ev2h_version(void) { return 102; }
 extern "C" const char *ev2h_last_error(void) { return ev2h::g_err; }

@@ -121,7 +121,7 @@ linear_relu_kernel(const float *__restrict__ x, int64_t M, int ld_x, int Cin,
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
                 const int n = n0 + h * 64 + tx * 4;
-                if (n + 3 < n_store && ((ld_y | y_col_off) & 3) == 0) {
+                if (n + 3 < n_store && ((ld_y | y_col_off) & 3) == 0 && ((uintptr_t)y & 15) == 0) {
                     *reinterpret_cast<float4 *>(yr + n) =
                         make_float4(acc[i][4 * h], acc[i][4 * h + 1], acc[i][4 * h + 2], acc[i][4 * h + 3]);
                 } else {

@@ -441,7 +441,7 @@ linear_tc_kernel(const TcParams p) {
                 if (K == 0) {
                     if (row_ok) {
                         float *yr = p.y + (m0 + r) * (int64_t)p.ld_y + p.y_col_off + col0 + c0;
-                        const bool vec = (((p.ld_y | p.y_col_off) & 3) == 0);
+                        const bool vec = (((p.ld_y | p.y_col_off) & 3) == 0) && ((uintptr_t)p.y & 15) == 0;
 #pragma unroll
                         for (int j = 0; j < 32; j += 4) {
                             if (vec && c0 + j + 3 < n_store) {

@@ -80,7 +80,7 @@ three_interp_kernel(const float *__restrict__ feats, int ld_f, const int32_t *__
         const float *f0 = feats + (b * S + id[0]) * (int64_t)ld_f + c, *f1 = feats + (b * S + id[1]) * (int64_t)ld_f + c,
                     *f2 = feats + (b * S + id[2]) * (int64_t)ld_f + c;
         float *o = out + r * (int64_t)ld_out + col + c;
-        if (c + 3 < D && (ld_f & 3) == 0 && ((ld_out | col) & 3) == 0) {
+        if (c + 3 < D && (ld_f & 3) == 0 && ((ld_out | col) & 3) == 0 && (((uintptr_t)feats | (uintptr_t)out) & 15) == 0) {
             const float4 a = *reinterpret_cast<const float4 *>(f0), bb = *reinterpret_cast<const float4 *>(f1),
                          cc = *reinterpret_cast<const float4 *>(f2);
             float4 v;

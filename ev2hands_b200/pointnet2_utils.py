@@ -1029,8 +1029,9 @@ class PointNetFeaturePropagation(nn.Module):
             d3, i3 = d3[..., :3], i3[..., :3]
             w = 1.0 / (d3 + 1e-8)
             w = w / w.sum(dim=2, keepdim=True)
+            # min(3, S) neighbours: with S = 2 both sources are interpolated
             nb = torch.gather(f2.unsqueeze(1).expand(B, N, S, f2.shape[-1]), 2,
-                              i3.unsqueeze(-1).expand(B, N, 3, f2.shape[-1]))
+                              i3.unsqueeze(-1).expand(B, N, i3.shape[-1], f2.shape[-1]))
             up = (nb * w.unsqueeze(-1)).sum(dim=2)
         h = up if points1 is None else torch.cat([points1.transpose(1, 2), up], dim=-1)
         if _TRAIN_ROWS:

@@ -215,7 +215,8 @@ EV2H_API int ev2h_fold_conv_bn_f32(const float *conv_w, const float *conv_b, con
  * ev2h_fold_conv_bn_f32.  pool_rows == 0: y is [M, ld_y].  pool_rows = K > 0 fuses
  * the max over each run of K consecutive rows (torch.max(x, 2)[0],
  * pointnet2_utils.py:257): y is [M/K, ld_y] written at column y_col_off and MUST be
- * zero-filled by the caller beforehand (post-ReLU values are >= 0).
+ * zero-filled by the caller beforehand (post-ReLU values are >= 0).  y needs only the
+ * alignment of a float.
  * argmax (optional, only with pool_rows) is not produced here; see
  * ev2h_group_max_f32 for the training path. */
 EV2H_API int ev2h_linear_relu_f32(const float *x, int64_t M, int ld_x, int Cin, const float *wt,
@@ -243,6 +244,12 @@ EV2H_API int ev2h_linear_f32(const float *x, int64_t M, int ld_x, int Cin, const
  * pool_rows must be 0, 32, 64 or a multiple of 128; Cout <= 256 or a multiple of 256;
  * other shapes return EV2H_ERR_UNSUPPORTED (callers use ev2h_linear_relu_f32 for those).
  * Columns Cin .. ld_x - 1 of x are padding and never enter the product, whatever they hold (NaN included).
+ * Output columns: without pooling (pool_rows == 0, ev2h_linear_tc, ev2h_conv1d_tc) the kernel writes columns
+ * y_col_off .. y_col_off + P - 1 of every row, where P = min(ld_y - y_col_off, Cout rounded up to the accumulator
+ * block: a multiple of 16 below 256 channels, of 256 above): the Cout results, then exact +0.0 in the padding
+ * columns.  A caller sizing rows to round_up(Cout, 4) gets those padding columns zeroed.  With pooling only the
+ * Cout result columns of each pooled row are written.  Every other column of y keeps what it held.
+ * x and w_packed must be 16-byte aligned; y needs only the alignment of a float.
  * range_flag (device int32, may be NULL; used with EV2H_TC_F16X3 only): bit 0 is set (atomic OR, never
  * cleared) when an input operand left the fp16 range (|x| >= 65520) or was NaN.  The caller also checks the
  * weights it packs: the kernels see them only as fp16 pairs. */
@@ -308,7 +315,9 @@ EV2H_API int ev2h_ball_query_compact_range_f32(const float *xyz, int64_t stride_
  * sequence counting as zero (the convolution's zero padding).  The shifted rows are gathered by the kernel's loaders;
  * no im2col buffer exists.  w_packed = ev2h_tc_pack_weights_kc image of the [taps * Cin, Cout] matrix whose row
  * t * Cin + ci is W[:, ci, t] (kc 32, row_align 16); post_scale / post_shift may be NULL.  taps in {1, 3, 5}.
- * Columns Cin .. ld_x - 1 of x_rows are padding and never enter the product; range_flag as for ev2h_linear_tc. */
+ * Columns Cin .. ld_x - 1 of x_rows are padding and never enter the product; range_flag, the output columns written
+ * (the Cout results plus exact-zero padding up to the accumulator block width) and the alignment rules as for
+ * ev2h_linear_tc. */
 EV2H_API int ev2h_conv1d_tc(const float *x_rows, int64_t M, int ld_x, int Cin, int taps, int rows_per_seq, const void *w_packed,
                             const float *bias, int Cout, int relu, const float *post_scale, const float *post_shift,
                             float *y, int ld_y, int y_col_off, int mode, int32_t *range_flag, ev2h_stream_t stream);
@@ -399,7 +408,8 @@ EV2H_API int ev2h_three_nn_f32(const float *xyz1, int64_t q_stride_b, int64_t q_
                                int B, int N, int S, int32_t *idx, float *weight, ev2h_stream_t stream);
 /* interpolated[b,n,:] = sum_k feats[b, idx[b,n,k], :] * weight[b,n,k]  (:301), written at column col
  * of out_rows [B*N, ld_out] (the concat with points1 happens by writing next to it).
- * feats_rows [B*S, ld_f], D channels. */
+ * feats_rows [B*S, ld_f], D channels.  Only columns col .. col + D - 1 of out_rows are written.  feats_rows and
+ * out_rows need only the alignment of a float. */
 EV2H_API int ev2h_three_interp_f32(const float *feats_rows, int ld_f, const int32_t *idx, const float *weight,
                                    int B, int N, int S, int D, float *out_rows, int ld_out, int col,
                                    ev2h_stream_t stream);

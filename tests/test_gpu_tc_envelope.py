@@ -238,7 +238,7 @@ def test_fused_envelope_vs_f64(name, mode, monkeypatch):
 TC_MODES = {"bf16": _capi.TC_BF16, "tf32x3": _capi.TC_TF32X3, "tf32_bf16c": _capi.TC_TF32_BF16C, "f16x3": _capi.TC_F16X3}
 # entry -> (taps, relu, pool_rows)
 ENTRIES = {"linear_tc": (1, False, 0), "linear_relu_tc": (1, True, 0), "linear_relu_tc_pool128": (1, True, 128),
-           "conv1d_tc_k1": (1, True, 0), "conv1d_tc_k3": (3, True, 0)}
+           "conv1d_tc_k1": (1, True, 0), "conv1d_tc_k3": (3, True, 0), "conv1d_tc_k5": (5, True, 0)}
 
 
 def _tol(tc_mode):
