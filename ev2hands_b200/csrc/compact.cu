@@ -138,9 +138,13 @@ first_occurrence_kernel(const float *__restrict__ pts8, int N, uint8_t *__restri
     uint8_t *out = first + (int64_t)blockIdx.x * N;
     for (int i = threadIdx.x; i < slots; i += kUniqThreads) table[i] = 0x7fffffff;
     __syncthreads();
+    // the hash covers all eight words: records of few features keep xyz in words 4..7, and records that differ only in
+    // unhashed words would all probe one chain (16384 such records: 258 ms with words 0..4 hashed, 0.14 ms with all
+    // eight, on a B200)
     auto slot_of = [&](int n) {
         const uint4 a = rec[2 * n], b = rec[2 * n + 1];
-        uint32_t h = a.x * 0x9E3779B1u ^ a.y * 0x85EBCA77u ^ a.z * 0xC2B2AE3Du ^ a.w * 0x27D4EB2Fu ^ b.x * 0x165667B1u;
+        uint32_t h = a.x * 0x9E3779B1u ^ a.y * 0x85EBCA77u ^ a.z * 0xC2B2AE3Du ^ a.w * 0x27D4EB2Fu ^ b.x * 0x165667B1u ^
+                     b.y * 0xD3A2646Du ^ b.z * 0xFD7046C5u ^ b.w * 0xB55A4F09u;
         h ^= h >> 15;
         return (int)(h & (slots - 1));
     };

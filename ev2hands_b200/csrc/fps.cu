@@ -49,6 +49,18 @@ __device__ __forceinline__ void unpack2(uint64_t v, float &a, float &b) { asm("m
 __device__ __forceinline__ uint64_t sub2(uint64_t a, uint64_t b) { uint64_t d; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 __device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) { uint64_t d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 __device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) { uint64_t d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+// (dx^2 + dy^2) + dz^2 for two points, every product and sum rounded, as torch.sum((xyz - centroid) ** 2, -1).
+// ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 despite the rounding modifier (also under --fmad=false), and
+// the fused sum breaks the reference's ties (tests/test_gpu_geometry_envelope.py, N = 8193).  Each square is
+// fma(d, d, -0) instead, which is round(d * d) exactly and leaves no multiply for the adds to absorb; the -0 comes from
+// constant memory, since ptxas folds a literal -0 addend back into a multiply (and then fuses again).
+__constant__ uint64_t kNegZero2 = 0x8000000080000000ull;     // -0.0f in both halves
+__device__ __forceinline__ uint64_t sq2(uint64_t a) {
+    uint64_t d; asm("fma.rn.f32x2 %0, %1, %1, %2;" : "=l"(d) : "l"(a), "l"(kNegZero2)); return d;
+}
+__device__ __forceinline__ void sqdist2(uint64_t dx, uint64_t dy, uint64_t dz, float &d0, float &d1) {
+    unpack2(add2(add2(sq2(dx), sq2(dy)), sq2(dz)), d0, d1);
+}
 }  // namespace cl
 
 template <int T, int P, int RP>      // RP = points per thread whose coordinates stay in registers (P: all; fewer for very long windows)
@@ -134,7 +146,7 @@ fps_kernel(const float *__restrict__ xyz, int64_t sb, int64_t sc, int64_t sn,
             }
             const uint64_t dx = cl::sub2(px2, cx2), dy = cl::sub2(py2, cy2), dz = cl::sub2(pz2, cz2);
             float d0, d1;
-            cl::unpack2(cl::add2(cl::add2(cl::mul2(dx, dx), cl::mul2(dy, dy)), cl::mul2(dz, dz)), d0, d1);   // (dx^2 + dy^2) + dz^2, un-fused
+            cl::sqdist2(dx, dy, dz, d0, d1);                                                               // (dx^2 + dy^2) + dz^2, un-fused
             const float m0 = d0 < best[j] ? d0 : best[j], m1 = d1 < best[j + 1] ? d1 : best[j + 1];          // distance[mask] = dist[mask], :81-82
             best[j] = m0; best[j + 1] = m1;
             const unsigned v0 = __float_as_uint(m0), v1 = __float_as_uint(m1);
@@ -238,7 +250,7 @@ fps_cluster_kernel(const float *__restrict__ xyz, int64_t sb, int64_t sc, int64_
         for (int j = 0; j < P; j += 2) {
             const uint64_t dx = cl::sub2(x2[j / 2], cx2), dy = cl::sub2(y2[j / 2], cy2), dz = cl::sub2(z2[j / 2], cz2);
             float d0, d1;
-            cl::unpack2(cl::add2(cl::add2(cl::mul2(dx, dx), cl::mul2(dy, dy)), cl::mul2(dz, dz)), d0, d1);   // (dx^2 + dy^2) + dz^2, un-fused
+            cl::sqdist2(dx, dy, dz, d0, d1);                                                               // (dx^2 + dy^2) + dz^2, un-fused
             const float m0 = d0 < best[j] ? d0 : best[j], m1 = d1 < best[j + 1] ? d1 : best[j + 1];          // distance[mask] = dist[mask], :81-82
             best[j] = m0; best[j + 1] = m1;
             const unsigned v0 = __float_as_uint(m0), v1 = __float_as_uint(m1);
@@ -528,7 +540,7 @@ fps_pruned_kernel(const float *__restrict__ xyz, int64_t sb, int64_t sc, int64_t
                         const uint64_t pz2 = cl::pack2(sz[p0 + k * 32], sz[p0 + k * 32 + 32]);
                         const uint64_t dx = cl::sub2(px2, cx2), dy = cl::sub2(py2, cy2), dz = cl::sub2(pz2, cz2);
                         float d0, d1;
-                        cl::unpack2(cl::add2(cl::add2(cl::mul2(dx, dx), cl::mul2(dy, dy)), cl::mul2(dz, dz)), d0, d1);   // (dx^2 + dy^2) + dz^2, un-fused
+                        cl::sqdist2(dx, dy, dz, d0, d1);                                                               // (dx^2 + dy^2) + dz^2, un-fused
                         best[q] = d0 < best[q] ? d0 : best[q];                                                           // distance[mask] = dist[mask], :81-82
                         best[q + 1] = d1 < best[q + 1] ? d1 : best[q + 1];
                     }
